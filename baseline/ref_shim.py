@@ -5,8 +5,8 @@ rvfm.py:8,65) and the HuggingFace hub (backbones.py:275,285 call `AutoModel/Auto
 shim registers a six-line `omegaconf` stub and replaces the three `from_pretrained` entry points with factories that
 build the same objects from the hub configs of facebook/deit-{tiny,small,base}-patch16-224 (model_type "vit":
 12 layers, patch 16, 224 px, gelu, qkv bias, eps 1e-12 = ViTConfig defaults; DeiT processor with the ImageNet
-mean / std).  The reference code itself is imported UNMODIFIED from baseline/_ref (pip-installed copy) or, in the
-build container, from /root/reference/src."""
+mean / std).  The reference code itself is imported UNMODIFIED from oracle/_ref (the pip-installed copy build()
+makes, oracle/install_ref.py) or, where only the source tree exists, from that tree."""
 from __future__ import annotations
 
 import os
@@ -24,7 +24,7 @@ IMAGE_STD = (0.229, 0.224, 0.225)
 
 
 def reference_path(prefer_installed: bool = True):
-    inst = os.path.join(HERE, "_ref")
+    inst = os.path.join(os.path.dirname(HERE), "oracle", "_ref")  # oracle/install_ref.py
     if prefer_installed and os.path.exists(os.path.join(inst, "theia", "models", "rvfm.py")):
         return inst
     if os.path.exists("/root/reference/src/theia/models/rvfm.py"):
@@ -66,8 +66,8 @@ def import_reference(prefer_installed: bool = True):
     """Returns the reference's RobotVisionFM class, or raises ImportError when no copy of the reference exists."""
     path = reference_path(prefer_installed)
     if path is None:
-        raise ImportError("no reference package: baseline/_ref is missing (run baseline/install_ref.py where "
-                          "/root/reference exists)")
+        raise ImportError("no reference package: oracle/_ref is missing (build() installs it where the reference's "
+                          "source tree is available)")
     install_shims()
     if path not in sys.path:
         sys.path.insert(0, path)

@@ -4,16 +4,18 @@
     python bench.py --gpus 1 --steps 20 --warmup 5
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
-    python bench.py --impl reference ...      # the UNMODIFIED reference (baseline/_ref) on the host cores
+    python bench.py --impl reference ...      # the UNMODIFIED reference (oracle/_ref) on the host cores
     python bench.py --impl eager ...          # the same reference modules through torch eager on one B200
 
 One step = train_rvfm.py:116-133 on one synthetic batch: forward (pre-process, DeiT student, lconv
 translator heads) -> get_loss -> main_loss = 0.9 cos + 0.1 smooth-l1 -> backward -> AdamW step,
-through the public `RobotVisionFM` API.  Prints ONE JSON line (rank 0).
+through the public `RobotVisionFM` API.  Prints ONE JSON line (rank 0).  --dump-outputs DIR also writes what the
+last timed step computed as DIR/*.npy (see dump_outputs), to compare two builds on identical seeded inputs.
 """
 from __future__ import annotations
 
 import argparse
+import copy
 import json
 import os
 import subprocess
@@ -132,7 +134,7 @@ def pick_cpu_threads(probe):
 
 
 def build_reference_module(cfgO, O, backbone, device):
-    """The UNMODIFIED reference `RobotVisionFM` (baseline/_ref, pip-installed copy of /root/reference) with the
+    """The UNMODIFIED reference `RobotVisionFM` (oracle/_ref, the pip-installed copy build() makes) with the
     oracle's deterministic weights, or None when that copy is absent."""
     try:
         from baseline import ref_shim
@@ -172,7 +174,7 @@ def reference_step_fn(ref, cfgO, O, B, device, autocast=False, lr=1e-4):
 
 def run_reference(args, cfgO, O):
     """The reference's own CPU implementation of the step on the host cores: the UNMODIFIED reference modules from
-    baseline/_ref (kind "reference"); the oracle port only when that copy is absent (kind "port")."""
+    oracle/_ref (kind "reference"); the oracle port only when that copy is absent (kind "port")."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -214,8 +216,8 @@ def run_reference(args, cfgO, O):
         step()
     dt = (time.perf_counter() - t0) / args.steps
     val = B / dt
-    what = ("UNMODIFIED reference RobotVisionFM (baseline/_ref) + torch AdamW, fp32 CPU" if kind == "reference"
-            else "oracle port (torch fp32 CPU; baseline/_ref absent)")
+    what = ("UNMODIFIED reference RobotVisionFM (oracle/_ref) + torch AdamW, fp32 CPU" if kind == "reference"
+            else "oracle port (torch fp32 CPU; oracle/_ref absent)")
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": "images/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt * 1e3, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -231,7 +233,7 @@ def run_reference(args, cfgO, O):
 def gpu_eager_leg(args, cfgO, O, dev, steps=3):
     """The meaningful GPU comparator (SURVEY 8d / BASELINE.md section 3): the reference's own modules run by torch
     eager (cuBLAS / cuDNN / ATen) on the SAME B200, same replayed step and batch, in fp32 (as the reference trains)
-    and under autocast(bfloat16).  Returns None when baseline/_ref is absent."""
+    and under autocast(bfloat16).  Returns None when oracle/_ref is absent."""
     out = {}
     for mode in ("fp32", "autocast_bf16"):
         ref = build_reference_module(cfgO, O, BACKBONES[args.backbone], dev)
@@ -255,7 +257,7 @@ def gpu_eager_leg(args, cfgO, O, dev, steps=3):
             out[mode] = {"value": None, "note": f"out of memory at batch {B}"}
         del ref
         torch.cuda.empty_cache()
-    out["what"] = ("UNMODIFIED reference RobotVisionFM (baseline/_ref) on this GPU through torch eager "
+    out["what"] = ("UNMODIFIED reference RobotVisionFM (oracle/_ref) on this GPU through torch eager "
                    "(cuBLAS/cuDNN/ATen), fwd+get_loss+bwd+torch AdamW; inputs copied from host each step as "
                    "train_rvfm.py:101-114 does; matmul TF32 off (torch default), cuDNN conv TF32 on (torch default)")
     return out
@@ -283,7 +285,7 @@ def cpu_baseline_leg(args, cfgO, O):
     for _ in range(nrep):
         step()
     dt = (time.perf_counter() - t0) / nrep
-    what = ("UNMODIFIED reference RobotVisionFM (baseline/_ref), fp32 CPU: fwd+loss+bwd+AdamW" if kind == "reference"
+    what = ("UNMODIFIED reference RobotVisionFM (oracle/_ref), fp32 CPU: fwd+loss+bwd+AdamW" if kind == "reference"
             else "oracle port (torch fp32 CPU): fwd+loss+bwd")
     return {"value": Bc / dt, "unit": "images/s", "cores": cores, "kind": kind,
             "sample": f"{what}, batch {Bc}, {nrep} timed steps; threads chosen from "
@@ -319,6 +321,44 @@ def parity_check(model, cfgO, O, d_images, d_targets, dev, n=4):
     return out
 
 
+DUMP_SAMPLE = 1 << 20  # elements kept of each large array (4 MiB each, 20 MiB for the three cdiv teachers)
+
+
+def dump_outputs(out_dir, model, last):
+    """What the last timed step handed its caller, as float32 / float64 .npy files: pred_<teacher> (predictions),
+    main_loss / mse_loss / cos_loss / l1_loss, loss_<teacher> (that teacher's mse, cos and l1 loss), grads (the
+    step's parameter gradients) and params (the parameters after the AdamW update), both in model.parameters() order.
+    That step starts from the seeded initial weights and optimizer state (see timed_step in main).
+    Arrays above DUMP_SAMPLE elements keep the same seeded sample of positions on every run, so that two builds can
+    be compared element by element."""
+    import numpy as np
+
+    def sample(t):
+        f = t.detach().flatten()
+        if f.numel() > DUMP_SAMPLE:
+            idx = torch.randint(0, f.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0))
+            f = f[idx.sort().values.to(f.device)]
+        return f.float().cpu().numpy()
+
+    def fname(t):
+        return t.replace("/", "_")
+
+    losses = last["losses"]
+    arrays = {"pred_" + fname(t): sample(v) for t, v in last["pred"].items()}
+    for k in ("main_loss", "mse_loss", "cos_loss", "l1_loss"):
+        arrays[k] = np.array(float(last["main_loss"] if k == "main_loss" else losses[k]), dtype=np.float64)
+    for t in last["pred"]:
+        arrays["loss_" + fname(t)] = np.array([losses[k + "_losses_per_model"][t] for k in ("mse", "cos", "l1")],
+                                              dtype=np.float64)
+    params = list(model.parameters())
+    arrays["grads"] = sample(torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).flatten()
+                                        for p in params]))
+    arrays["params"] = sample(torch.cat([p.detach().flatten() for p in params]))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload_config(args, B):
     return {"workload": f"theia-{args.backbone} {args.teachers} distill step (fwd+loss+bwd+AdamW), per-GPU batch {B}, "
                         f"224x224x3 uint8 -> {args.teachers} teacher targets",
@@ -350,20 +390,26 @@ def main():
     ap.add_argument("--optimizer", default="flat", choices=["flat", "torch"],
                     help="flat = theia_b200.optim.FlatAdamW (one fused pass over the flat buffers); torch = torch.optim.AdamW(fused=True)")
     ap.add_argument("--gemm-csv", default=None, help="dump per-launch GEMM timings of the timed region")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step computed (predictions, losses, gradients, updated "
+                         "parameters; fixed seeded samples of the large arrays) as DIR/<name>.npy; that step "
+                         "starts from the seeded initial weights and optimizer state")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
 
     from oracle import theia_oracle as O  # checker / CPU baseline only
     cfgO = O.make_config(BACKBONES[args.backbone], args.teachers)
     if args.impl == "reference":
-        if args.steps > 5:
-            args.steps = max(1, min(args.steps, 5))  # bounded sample: the whole run must end within minutes
         args.warmup = min(args.warmup, 1)
         run_reference(args, cfgO, O)
         return
     if args.impl == "eager":
         if int(os.environ.get("RANK", "0")) == 0:
             torch.cuda.set_device(0)
-            eg = gpu_eager_leg(args, cfgO, O, torch.device("cuda", 0), steps=max(1, min(args.steps, 5)))
+            eg = gpu_eager_leg(args, cfgO, O, torch.device("cuda", 0), steps=args.steps)
             print(json.dumps({"impl": "eager", "metric": METRIC, "unit": "images/s", "n_gpus": 1,
                               "config": workload_config(args, args.batch), "gpu_eager_baseline": eg}), flush=True)
         return
@@ -416,6 +462,8 @@ def main():
     d_images = h_images.to(dev)
     d_targets = {t: v.to(dev) for t, v in h_targets.items()}
 
+    last = {}  # the last step's results, kept only for --dump-outputs
+
     def step(images, targets):
         pred = net(images, do_resize=False)
         losses = model.get_loss(pred, targets)  # returns python floats per teacher (one D2H), like the reference
@@ -423,6 +471,8 @@ def main():
         opt.zero_grad(set_to_none=True)
         main_loss.backward()
         opt.step()
+        if args.dump_outputs:
+            last.update(pred=pred, losses=losses, main_loss=main_loss)
         return losses
 
     def barrier():
@@ -445,6 +495,9 @@ def main():
             ms = float(t)
         return ms
 
+    start = None
+    if args.dump_outputs:  # the state the first step starts from
+        start = (model._flat.detach().clone(), copy.deepcopy(opt.state_dict()))
     parity = None
     if rank == 0 and not args.no_parity:
         parity = parity_check(model, cfgO, O, d_images, d_targets, dev)
@@ -454,7 +507,33 @@ def main():
     sampler = ClockSampler(local) if rank == 0 else None
     n0 = lib.theia_launch_count()
     _lib.check(lib.theia_prof_enable(1))
-    ms = timed(lambda i: step(d_images, d_targets), args.steps)
+
+    reset = []
+
+    def timed_step(i):
+        if start is not None and i == args.steps - 1:
+            # the fp32 atomics of the CUDA path sum in a different order on each run and every AdamW step on the
+            # synthetic batch amplifies that noise, so the step whose outputs are dumped starts again from the
+            # seeded initial weights and a fresh optimizer: its inputs are then identical from run to run.  The
+            # restore and the re-pack of the restored weights are timed apart and left out of `value`.
+            reset[:] = [torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)]
+            reset[0].record()
+            with torch.no_grad():
+                model._flat.copy_(start[0])
+            opt.load_state_dict(start[1])
+            model._ensure(B)
+            reset[1].record()
+        step(d_images, d_targets)
+
+    ms = timed(timed_step, args.steps)
+    reset_ms = reset[0].elapsed_time(reset[1]) if reset else 0.0  # timed() ended in a synchronize
+    if world > 1:
+        t = torch.tensor([reset_ms], device=dev)
+        dist.all_reduce(t, op=dist.ReduceOp.MIN)
+        reset_ms = float(t)
+    ms -= reset_ms
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, last)  # before the e2e leg steps the model further
     import ctypes as C
     pm, pf, pn = C.c_double(), C.c_double(), C.c_longlong()
     if args.gemm_csv and rank == 0:
@@ -551,6 +630,10 @@ def main():
             "vs_baseline": None, "dtype": "bf16", "data": "synthetic", "config": workload_config(args, B),
             "clocks": clocks, "e2e": e2e, "gpu_launches": int(launches), "roofline": roofline, "cpu_baseline": cpu,
             "gpu_eager_baseline": eager, "parity_check": parity}
+    if args.dump_outputs:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "reset_ms_excluded": reset_ms,
+                                "note": "the last timed step started from the seeded initial weights and optimizer "
+                                        "state; restoring them took reset_ms_excluded, left out of value"}
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -29,7 +29,8 @@ def import_reference():
 
 
 def sl(t: torch.Tensor) -> torch.Tensor:
-    """strided sample that keeps fixtures small"""
+    """strided sample that keeps fixtures small (tests/test_oracle.py and tests/test_teachers_gpu.py repeat it as
+    _sl: the three must stay identical)"""
     f = t.detach().flatten()
     step = max(1, f.numel() // 4096)
     return f[::step][:4096].clone()
@@ -125,6 +126,8 @@ def main():
 
     if not only or "tiny_anysize" in only:
         anysize(RobotVisionFM)
+    if not only or "teachers" in only:
+        teachers()
     if only and "readme_zeros" not in only:
         return
     # README quick-start (BASELINE config #1): zeros image through deit-tiny forward_feature
@@ -176,6 +179,25 @@ def anysize(RobotVisionFM):
         print(f"anysize {H}x{W} do_resize={do_resize}: oracle == reference, |f| = {float(f.abs().mean()):.4f}")
     path = os.path.join(os.path.dirname(HERE), "tests", "golden", "anysize_tiny.pt")
     torch.save({"case": "tiny_anysize", "cases": out}, path)
+    print("->", path, f"({os.path.getsize(path) / 1024:.0f} KiB)")
+
+
+def teachers():
+    """the reference's teacher wrappers (get_dinov2_feature / get_clip_feature / get_vit_feature) on the seeded HF
+    models and images of tests/test_teachers_gpu.py, fp32 on CPU; the summaries become tests/golden/teachers.pt"""
+    from theia.foundation_models.vision_language_models.clip import get_clip_feature
+    from theia.foundation_models.vision_models.dinov2 import get_dinov2_feature
+    from theia.foundation_models.vision_models.vit import get_vit_feature
+    from tests._teacher_util import CASES, _build, _images, _processors, _randomize
+    fns = {"dinov2": get_dinov2_feature, "clip": get_clip_feature, "vit": get_vit_feature}
+    out = []
+    for kind, arch, B in CASES:
+        hf = _randomize(_build(kind, arch), seed=1)
+        want = fns[kind](hf, _processors()[kind], _images(B))
+        out.append({"kind": kind, "arch": arch, "B": B, "outputs": [summarize(w) for w in want]})
+        print(f"teacher {kind} {arch} B={B}: {[tuple(w.shape) for w in want]}")
+    path = os.path.join(os.path.dirname(HERE), "tests", "golden", "teachers.pt")
+    torch.save({"case": "teachers", "cases": out, "versions": {"torch": torch.__version__}}, path)
     print("->", path, f"({os.path.getsize(path) / 1024:.0f} KiB)")
 
 

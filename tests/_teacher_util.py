@@ -1,8 +1,29 @@
 """HF teacher architectures with seeded random weights + the processors of the real checkpoints (offline)."""
 import math
 
+import numpy as np
 import torch
 import torch.nn.functional as F
+
+
+# (kind, (hidden, heads, layers, patch), batch) of tests/test_teachers_gpu.py and tests/golden/teachers.pt
+CASES = [
+    ("dinov2", (1024, 16, 24, 14), 3),  # facebook/dinov2-large: 257 tokens
+    ("dinov2", (384, 6, 12, 14), 5),    # facebook/dinov2-small
+    ("clip", (1024, 16, 24, 14), 2),    # openai/clip-vit-large-patch14: quick_gelu, pre_layrnorm, post_layernorm(cls)
+    ("clip", (768, 12, 12, 16), 4),     # openai/clip-vit-base-patch16: 197 tokens (the student's attention kernel)
+    ("vit", (768, 12, 12, 16), 3),      # google/vit-base-patch16-224-in21k
+    ("vit", (1024, 16, 4, 14), 2),      # ViT-L/14 geometry, shortened
+    ("vit", (1280, 16, 32, 14), 2),     # google/vit-huge-patch14-224-in21k (the reference's default): head dim 80
+]
+
+
+def _images(B):
+    """B seeded uint8 HWC images, the first one constant (all zeros)"""
+    rng = np.random.default_rng(3)
+    images = [rng.integers(0, 256, (224, 224, 3), dtype=np.uint8) for _ in range(B)]
+    images[0][:] = 0
+    return images
 
 
 def _randomize(model, seed):

@@ -1,5 +1,5 @@
 """The reference's OWN training loop (`theia/scripts/train/train_rvfm.py::train`, lines 38-208, imported unmodified
-from baseline/_ref) driving `theia_b200.RobotVisionFM`: DDP wrap (train_rvfm.py:258), the reference's parameter
+from oracle/_ref) driving `theia_b200.RobotVisionFM`: DDP wrap (train_rvfm.py:258), the reference's parameter
 groups (optimizers/utils.py:8-35), torch AdamW, the reference's LR scheduler (lr_schedulers.py:41-77), train + eval
 epochs, `freeze_translator()` at the configured step ratio (:149-151), gradient clipping (:126-130), checkpoint saves (:153-156, :203-206).
 
@@ -25,7 +25,7 @@ class _NS(types.SimpleNamespace):
 def _import_reference_train():
     from baseline import ref_shim
     if ref_shim.reference_path() is None:
-        pytest.skip("baseline/_ref (pip-installed copy of the reference) is not present")
+        pytest.skip("oracle/_ref (pip-installed copy of the reference, made by build()) is not present")
     ref_shim.install_shims()
     path = ref_shim.reference_path()
     if path not in sys.path:
